@@ -77,6 +77,23 @@ def env_int(k, d):
     return int(os.environ.get(k, d))
 
 
+DUMP_LIMIT = 60 << 20  # data budget of --dump-outputs: with the .npy headers the files stay under 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: writes the arrays a caller of the timed path received from its last step as <out_dir>/<name>.npy, floating point as
+    float32 (float64 stays float64), integers as float64 (exact).  An array larger than its share of DUMP_LIMIT is stored as every k-th
+    element of the flattened array, k the smallest stride that fits, so that two builds can be compared output for output."""
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_LIMIT // len(arrays)
+    for name, t in arrays.items():
+        t = t.detach()
+        a = (t.float() if t.is_floating_point() and t.dtype != torch.float64 else t.double()).cpu().numpy()
+        if a.nbytes > share:
+            a = a.reshape(-1)[::-(-a.nbytes // share)]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
+
+
 # ------------------------------------------------------------------------------------------------ clocks
 class ClockSampler:
     def __init__(self, gpu_index):
@@ -360,6 +377,8 @@ def run_b200_arm(args):
     barrier()
     total_ms = max_over_ranks(t_start.elapsed_time(t_end))
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # before the eager passes below overwrite the graph's output buffers
+        dump_outputs(args.dump_outputs, {'det': ws.det, 'det_idx': ws.det_idx, 'det_count': ws.det_count})
     ms_per_step = total_ms / K
     value = world * B * K / (total_ms / 1e3)
     launches = _lib.launch_count() - n0
@@ -604,6 +623,9 @@ def run_secondary_arm(args):
     total_ms = max_over_ranks(t0.elapsed_time(t1))
     clocks = sampler.stop() if rank == 0 else None
     value = world * B * K / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:  # before g.run() below overwrites the graph's output buffers
+        names = {'fcos': ('scores', 'classes', 'boxes', 'count'), 'deeplab': ('labels',), 'yolox': ('det', 'count')}[name]
+        dump_outputs(args.dump_outputs, dict(zip(names, results())))
     n1 = _lib.launch_count()
     g.run()
     torch.cuda.synchronize()
@@ -800,6 +822,8 @@ def run_train_arm(args):
     t1.record()
     barrier()
     total_ms = max_over_ranks(t0.elapsed_time(t1))
+    if args.dump_outputs and rank == 0:  # the block's parameters and BatchNorm statistics after the last step, before eager_step(0) below
+        dump_outputs(args.dump_outputs, m.state_dict())
     n0 = _lib.launch_count()
     eager_step(0)  # (counts the library launches of one step; graph replays do not pass through the C ABI)
     torch.cuda.synchronize()
@@ -929,7 +953,7 @@ def run_train_arm(args):
 def run_train_reference_arm(args):
     if env_int('RANK', 0) != 0:
         return
-    steps = max(1, min(args.steps, 5))
+    steps = args.steps
     v, cores, spt, sample = _train_cpu(steps)
     line = {'impl': 'reference', 'metric': TRAIN_CFG['metric'], 'value': round(v, 4), 'unit': 'images/sec', 'n_gpus': args.gpus, 'steps': steps, 'warmup': 1,
             'ms_per_step': round(spt * 1e3, 3), 'higher_is_better': True, 'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
@@ -957,7 +981,8 @@ def run_secondary_reference_arm(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=100)
+    ap.add_argument('--steps', type=int, default=None, help='timed steps (default: 100 for yolov5s and the --impl reference arms of the other '
+                    'inference configurations, 10 for fcos / deeplab / yolox, 20 for c3train, 5 for the c3train --impl reference arm)')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--config', default='yolov5s', choices=['yolov5s', 'c3train'] + sorted(SECONDARY),
@@ -968,14 +993,23 @@ def main():
     ap.add_argument('--graph', type=int, default=1, help='1 (default): the timed steps replay captured CUDA graphs (the conv-stack time for the roofline '
                     'comes from the conv launches replayed as their own graph); 0: eager launches with per-conv-segment events inside the timed region')
     ap.add_argument('--cpu-steps', type=int, default=3, help='CPU baseline steps timed on rank 0 (0 = skip)')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='after the timed steps, write the outputs of the last timed step to DIR/<name>.npy '
+                    '(rank 0; float32 / float64, at most 64 MB in all)')
     args = ap.parse_args()
+    if args.steps is None:  # the secondary GPU steps are 10-50 ms each, the CPU training step takes seconds
+        if args.config == 'c3train':
+            args.steps = 5 if args.impl == 'reference' else 20
+        else:
+            args.steps = 100 if (args.config == 'yolov5s' or args.impl == 'reference') else 10
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        ap.error('--dump-outputs writes the outputs of the B200 path (--impl b200)')
     if args.config == 'c3train':
         if args.impl == 'reference':
             return run_train_reference_arm(args)
         if not torch.cuda.is_available():
             raise SystemExit('bench.py: no CUDA device; the B200 path has no CPU fallback (use --impl reference for the CPU arm)')
-        if args.steps == 100:
-            args.steps = 20
         args.cpu_steps = min(args.cpu_steps, 3)
         return run_train_arm(args)
     if args.config == 'yolov5s':
@@ -985,8 +1019,6 @@ def main():
     else:
         if args.impl == 'reference':
             return run_secondary_reference_arm(args)
-        if args.steps == 100:
-            args.steps = 10  # the secondary steps are 10-50 ms each
         args.cpu_steps = min(args.cpu_steps, 2)
     if not torch.cuda.is_available():
         raise SystemExit('bench.py: no CUDA device; the B200 path has no CPU fallback (use --impl reference for the CPU arm)')

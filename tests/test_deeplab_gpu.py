@@ -70,7 +70,7 @@ def test_deeplab_forward_vs_reference_golden(cuda):
     assert labels.dtype == torch.int64 and tuple(labels.shape) == (2, 128, 256)
     G = model._graph_for(x, (128, 256))
     errs = {'low': _rel(ops.split_to_nchw(G['feats'][0].view())[:, ::8], g['low_sub']),
-            'high': _rel(ops.split_to_nchw(G['feats'][1].view()), g['high']),
+            'high': _rel(ops.split_to_nchw(G['feats'][1].view())[:, ::3], g['high']),
             'logits': _rel(G['logits'].data[..., :19].permute(0, 3, 1, 2), g['logits'])}
     print(errs)
     assert max(errs.values()) < TOL, errs

@@ -22,7 +22,7 @@ def test_deeplab_oracle_matches_reference():
     x = torch.randn(2, 3, 128, 256)
     feats, logits, labels = DO.forward(x, synth.deeplab_state_dict(True))
     rel = lambda a, b: float((a.double() - torch.from_numpy(b).double()).abs().max() / (np.abs(b).max() + 1e-12))
-    assert rel(feats[0][:, ::8], g['low_sub']) < 1e-5 and rel(feats[1], g['high']) < 1e-5 and rel(logits, g['logits']) < 1e-5
+    assert rel(feats[0][:, ::8], g['low_sub']) < 1e-5 and rel(feats[1][:, ::3], g['high']) < 1e-5 and rel(logits, g['logits']) < 1e-5
     assert float((labels.numpy() == g['labels']).mean()) > 0.9999  # exact unless a 1e-6 logit tie flips across CPUs
 
 

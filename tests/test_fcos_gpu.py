@@ -95,7 +95,7 @@ def test_fcos_forward_vs_reference_golden_128(model):
     torch.cuda.synchronize()
     G = model._graph_for(x)
     from cvpytorch_b200 import ops
-    errs = {'C5': _rel(ops.split_to_nchw(G['feats'][2].view()), g['C5'])}
+    errs = {'C5': _rel(ops.split_to_nchw(G['feats'][2].view())[:, ::3], g['C5'])}  # the fixture keeps every 3rd C5 channel
     for i in range(5):
         errs[f'P{i + 3}'] = _rel(ops.split_to_nchw(G['levels'][i].view()), g[f'P{i + 3}'])
         cls, rc = G['head'][i]
@@ -112,7 +112,7 @@ def test_fcos_components_nchw_api(model):
     torch.manual_seed(1029)
     x = torch.randn(2, 3, 128, 128).cuda()
     feats = model.backbone(x)
-    assert _rel(feats[2], g['C5']) < TOL
+    assert _rel(feats[2][:, ::3], g['C5']) < TOL
     levels = model.neck(feats)
     cls, cnt, reg = model.head(levels)
     for i in range(5):

@@ -31,7 +31,7 @@ def test_fcos_oracle_forward_matches_reference(sd):
     x = torch.randn(2, 3, 128, 128)
     feats, levels, cls, cnt, reg = FO.forward(x, sd)
     rel = lambda a, b: float((a.double() - torch.from_numpy(b).double()).abs().max() / (np.abs(b).max() + 1e-12))
-    assert rel(feats[2], g['C5']) < 1e-5
+    assert rel(feats[2][:, ::3], g['C5']) < 1e-5  # the fixture keeps every 3rd C5 channel
     for i in range(5):
         assert rel(levels[i], g[f'P{i + 3}']) < 1e-5 and rel(cls[i], g[f'cls{i}']) < 1e-5
         assert rel(cnt[i], g[f'cnt{i}']) < 1e-5 and rel(reg[i], g[f'reg{i}']) < 1e-5

@@ -6,6 +6,7 @@ Tolerances (bf16 step: 8-bit mantissa, |rounding| <= 2^-9 = 2e-3 per stored acti
   single kernels, bf16 outputs        max|a-b| / max|b| <= 6e-3        fp32 outputs (wgrad, BN statistics)  <= 2e-3
   whole block vs the fp32 reference   forward <= 3e-2, d/dx and every parameter gradient <= 6e-2  (5-9 bf16 layers deep each way)"""
 import os
+import sys
 
 import numpy as np
 import pytest
@@ -13,7 +14,9 @@ import torch
 import torch.nn.functional as F
 
 pytestmark = pytest.mark.gpu
-GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+GOLD = os.path.join(ROOT, 'tests', 'golden')
+sys.path.insert(0, os.path.join(ROOT, 'tools'))
 
 
 def _rel(a, b):
@@ -91,25 +94,26 @@ def test_bn_silu_forward_backward_and_fused_silu_grad_epilogue(cuda):
 @pytest.mark.parametrize('case', ['c3_n1', 'c3_n2'])
 def test_c3_training_step_vs_reference_fixture(cuda, case):
     from cvpytorch_b200 import train as T
+    from make_golden_train import case_inputs, sub
     g = np.load(os.path.join(GOLD, 'c3_train.npz'))
     cin, cout, n, B, H, W = [int(v) for v in g[f'{case}_cfg']]
     m = T.CSPLayer(cin, cout, n=n)
     keys = [str(k) for k in g[f'{case}_keys']]
     assert list(m.state_dict().keys()) == keys  # same module tree / parameter names as the reference block
-    m.load_state_dict({k: torch.from_numpy(g[f'{case}_sd_{k}']) for k in keys})
+    sd, x, G = case_inputs(case, m.state_dict())
+    m.load_state_dict(sd)
     for mod in m.modules():
         if isinstance(mod, torch.nn.BatchNorm2d):
             mod.eps, mod.momentum = 1e-3, 0.03
     m.cuda().train()
-    x = torch.from_numpy(g[f'{case}_x']).cuda().requires_grad_(True)
-    G = torch.from_numpy(g[f'{case}_G']).cuda()
+    x = x.cuda().requires_grad_(True)
     y = m(x)
-    (y * G).sum().backward()
+    (y * G.cuda()).sum().backward()
     torch.cuda.synchronize()
-    errs = {'y': _rel(y, torch.from_numpy(g[f'{case}_y'])), 'dx': _rel(x.grad, torch.from_numpy(g[f'{case}_dx']))}
+    errs = {'y': _rel(sub(y), torch.from_numpy(g[f'{case}_y'])), 'dx': _rel(sub(x.grad), torch.from_numpy(g[f'{case}_dx']))}
     for k, p in m.named_parameters():
         assert p.grad is not None, k
-        errs['grad ' + k] = _rel(p.grad, torch.from_numpy(g[f'{case}_grad_{k}']))
+        errs['grad ' + k] = _rel(sub(p.grad), torch.from_numpy(g[f'{case}_grad_{k}']))
     for k, v in m.state_dict().items():
         if 'running_' in k:
             errs['after ' + k] = _rel(v, torch.from_numpy(g[f'{case}_after_{k}']))
@@ -192,24 +196,25 @@ def test_stride2_conv_forward_backward_data_backward_weight(cuda, B, H, W, cin, 
 def test_dark_stage_training_step_vs_reference_fixture(cuda):
     """stride-2 BaseConv + CSPLayer (one `dark` stage) forward + backward vs the reference modules + torch.autograd (fixture case 'dark')."""
     from cvpytorch_b200 import train as T
+    from make_golden_train import case_inputs, sub
     g = np.load(os.path.join(GOLD, 'c3_train.npz'))
     down, csp = T.BaseConv(64, 128, 3, 2), T.CSPLayer(128, 128, n=1)
     m = torch.nn.Sequential(down, csp)
     keys = [str(k) for k in g['dark_keys']]
     assert list(m.state_dict().keys()) == keys
-    m.load_state_dict({k: torch.from_numpy(g[f'dark_sd_{k}']) for k in keys})
+    sd, x, G = case_inputs('dark', m.state_dict())
+    m.load_state_dict(sd)
     for mod in m.modules():
         if isinstance(mod, torch.nn.BatchNorm2d):
             mod.eps, mod.momentum = 1e-3, 0.03
     m.cuda().train()
-    x = torch.from_numpy(g['dark_x']).cuda().requires_grad_(True)
-    G = torch.from_numpy(g['dark_G']).cuda()
+    x = x.cuda().requires_grad_(True)
     y = csp.forward_nhwc(down(x.permute(0, 2, 3, 1).contiguous().to(torch.bfloat16))).permute(0, 3, 1, 2).float()
-    (y * G).sum().backward()
+    (y * G.cuda()).sum().backward()
     torch.cuda.synchronize()
-    errs = {'y': _rel(y, torch.from_numpy(g['dark_y'])), 'dx': _rel(x.grad, torch.from_numpy(g['dark_dx']))}
+    errs = {'y': _rel(sub(y), torch.from_numpy(g['dark_y'])), 'dx': _rel(sub(x.grad), torch.from_numpy(g['dark_dx']))}
     for k, p in m.named_parameters():
-        errs['grad ' + k] = _rel(p.grad, torch.from_numpy(g[f'dark_grad_{k}']))
+        errs['grad ' + k] = _rel(sub(p.grad), torch.from_numpy(g[f'dark_grad_{k}']))
     for k, v in m.state_dict().items():
         if 'running_' in k:
             errs['after ' + k] = _rel(v, torch.from_numpy(g[f'dark_after_{k}']))

@@ -32,6 +32,7 @@ def test_yolox_forward_matches_reference_fixture():
     for name, ts in (('backbone', b), ('neck', n), ('head', o)):
         for i, t in enumerate(ts):
             ref = g[f'{name}{i}']
+            t = t if name == 'backbone' else t[:, ::3]  # the fixture keeps every 3rd neck / head channel
             assert t.shape == ref.shape
             err = float(np.abs(t.numpy() - ref).max() / (np.abs(ref).max() + 1e-12))
             assert err <= 2e-5, (name, i, err)  # bit-identical in the build container; other CPUs/BLAS differ in the last bits

@@ -8,7 +8,7 @@ m = synth.build_yolov5s(True)
 rel = lambda a, b: float((a.double().cpu() - torch.as_tensor(b).double()).abs().max() / (np.abs(b).max() + 1e-12))
 g = np.load(os.path.join(ROOT, 'tests/golden/yolov5s_fwd128.npz'))
 torch.manual_seed(1029); x = torch.randn(2, 3, 128, 128).cuda()
-m.predict(x); e128 = rel(m._graph_for(x)['z'], g['z'])
+m.predict(x); e128 = rel(m._graph_for(x)['z'][:, ::3], g['z'])
 g = np.load(os.path.join(ROOT, 'tests/golden/yolov5s_fwd640.npz'))
 torch.manual_seed(1029); x = torch.randn(1, 3, 640, 640).cuda()
 m.predict(x); e640 = rel(m._graph_for(x)['z'][0, ::16], g['z_sub'])

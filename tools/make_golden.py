@@ -5,7 +5,7 @@ Run once in the build container:  python tools/make_golden.py
 
 Outputs
   yolov5s_calib.npz   BN running statistics + Detect scales of the calibrated synthetic model (see cvpytorch_b200/synth.py)
-  yolov5s_fwd128.npz  reference forward, 2x3x128x128 (seed 1029): backbone outs, neck outs, decoded z
+  yolov5s_fwd128.npz  reference forward, 2x3x128x128 (seed 1029): backbone outs, neck outs, decoded z (every 3rd channel / anchor row of each)
   yolov5s_fwd640.npz  reference forward, 1x3x640x640 (seed 1029): every 16th anchor row of z + reference NMS result on the full z
   nms_stress.npz      reference non_max_suppression (+torchvision.ops.nms) kept rows on the seeded stress set (4 regimes x 2 modes)
 """
@@ -94,8 +94,8 @@ def main():
     b, n, z, raws = ref_forward(x128)
     oz, oraws = YO.forward(x128, sd)
     print('oracle vs reference @128: z rel err', YO.rel_err(oz, z))
-    np.savez_compressed(os.path.join(GOLD, 'yolov5s_fwd128.npz'), z=z.numpy(), **{f'backbone{i}': t.numpy() for i, t in enumerate(b)},
-                        **{f'neck{i}': t.numpy() for i, t in enumerate(n)})
+    np.savez_compressed(os.path.join(GOLD, 'yolov5s_fwd128.npz'), z=z[:, ::3].numpy(), **{f'backbone{i}': t[:, ::3].numpy() for i, t in enumerate(b)},
+                        **{f'neck{i}': t[:, ::3].numpy() for i, t in enumerate(n)})
 
     torch.manual_seed(1029)
     x640 = torch.randn(1, 3, 640, 640)

@@ -3,7 +3,7 @@
 Run once in the build container:  python tools/make_golden_fcos.py
   fcos_keys.npz     state_dict keys/shapes of the reference ResNet / FCOSFPN / FCOSHead
   fcos_calib.npz    BN running statistics of the calibrated synthetic ResNet-50 + head scales (see cvpytorch_b200/synth.py)
-  fcos_fwd128.npz   reference forward, 2x3x128x128 (seed 1029): C5, P3..P7, per-level cls / cnt / reg
+  fcos_fwd128.npz   reference forward, 2x3x128x128 (seed 1029): every 3rd channel of C5, P3..P7, per-level cls / cnt / reg
   fcos_det256.npz   reference FCOSDetect on the reference's own head outputs, 1x3x256x256: scores / classes / boxes
   fcos_nms_stress.npz  reference _post_process (batched_nms + box_nms) on seeded synthetic candidates
 """
@@ -107,7 +107,7 @@ def main():
     ofe, olv, ocls, ocnt, oreg = FO.forward(x128, sd)
     errs = [float((a - b).abs().max() / b.abs().max()) for a, b in zip(list(ofe) + list(olv) + ocls + ocnt + oreg, list(feats) + list(levels) + cls + cnt + reg)]
     print('oracle vs reference @128 max rel err over all tensors:', max(errs))
-    out = {'C5': feats[2].numpy()}
+    out = {'C5': feats[2][:, ::3].numpy()}
     for i in range(5):
         out[f'P{i + 3}'] = levels[i].numpy()
         out[f'cls{i}'] = cls[i].numpy()

@@ -2,7 +2,7 @@
 
   yolox_keys.npz     state_dict keys / shapes of the reference composite (CSPDarknet + YOLOXNeck + YOLOXHead, SURVEY.md 3.5 row 3)
   yolox_calib.npz    BN running statistics of the calibration pass + predictor scales (cvpytorch_b200/synth.py)
-  yolox_fwd128.npz   reference forward at 2x3x128x128 (seed 1029): backbone / neck / head outputs
+  yolox_fwd128.npz   reference forward at 2x3x128x128 (seed 1029): backbone outputs, every 3rd channel of the neck / head outputs
   yolox_post320.npz  reference forward + yolox_post_process at 1x3x320x320: decoded tensor sample, detections
   yolox_nms.npz      reference yolox_post_process tail (score filter + torchvision.ops.batched_nms) on seeded candidate records,
                      both batched_nms regimes
@@ -124,7 +124,7 @@ def main():
     oo = XO.forward(x128, sd)
     print('oracle vs reference @128: head rel err', max(float((a - r).abs().max() / r.abs().max()) for a, r in zip(oo, o)))
     np.savez_compressed(os.path.join(GOLD, 'yolox_fwd128.npz'), **{f'backbone{i}': t.numpy() for i, t in enumerate(b)},
-                        **{f'neck{i}': t.numpy() for i, t in enumerate(n)}, **{f'head{i}': t.numpy() for i, t in enumerate(o)})
+                        **{f'neck{i}': t[:, ::3].numpy() for i, t in enumerate(n)}, **{f'head{i}': t[:, ::3].numpy() for i, t in enumerate(o)})
 
     torch.manual_seed(1029)
     x320 = torch.randn(1, 3, 320, 320)
